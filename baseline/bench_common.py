@@ -76,6 +76,9 @@ def parse_args(argv=None):
     p.add_argument("--clients-per-round", type=int, default=None, help="default: the BASELINE config's value")
     p.add_argument("--sync-ckpt", action="store_true", help="ours only: write latest_model.tar synchronously every "
                    "round like the reference (default: async latest-wins writer)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None, help="ours only: after the timed rounds write the "
+                   "last one's results (train loss, global model) to DIR/<name>.npy; set-up then runs a fixed number "
+                   "of rounds so the inputs of every round are the same on every run")
     args = p.parse_args(argv)
     if args.steps is None:
         args.steps = 20 if args.impl == "reference" else (200 if args.task in ("cv_resnet_fedcifar100", "cv_lr_mnist") else 40)

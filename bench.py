@@ -25,6 +25,16 @@ What is measured (all through the public API ``OptimizationServer.begin_training
 * ``--sync-ckpt`` writes ``latest_model.tar`` synchronously every round like the reference (default: async
   latest-wins writer); ``--norm bn`` runs the reference's as-shipped BatchNorm variant of the model.
 
+``--dump-outputs DIR`` writes what the last timed round returned to its caller, for comparing two builds output for
+output: ``train_loss.npy`` (float64, the loss ``run_rounds`` returned) and ``global_model.npy`` (float32, every
+floating-point tensor of the updated global model's state dict, flattened in order; a model of more than
+``DUMP_MAX_VALUES`` entries is written as a fixed, seeded sample of them).  Data, model init and client sampling are
+seeded and the set-up phase runs a fixed ``SETUP_ROUNDS_FIXED`` rounds, so every round has the same index and client
+sample on every run.  The last timed round also starts from the seeded initial global model, copied back in place
+before it: float atomics reorder the gradient sums of every earlier round, and training (GroupNorm over 2-channel
+groups on 1x1 maps) amplifies those last-bit differences round after round, so the weights it would otherwise start
+from differ between runs.  The dumped round thus has the same inputs on every run.
+
 ``gpu_launches`` counts launches of this repo's own kernels in the timed region (rank 0).
 ``FLUTE_BENCH_CPU=1`` runs the same protocol on CPU/gloo with a tiny population (control-flow test, no number).
 """
@@ -34,6 +44,9 @@ import sys
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "baseline"))
 from bench_common import (BASELINE_PUBLISHED, TASKS, ClockSampler, emit, parse_args)  # noqa: E402
+
+SETUP_ROUNDS_FIXED = 8              # with --dump-outputs; _settle() usually stops after 4-5 rounds
+DUMP_MAX_VALUES = 15_000_000        # float32 entries of global_model.npy: 60 MB, keeps a dump under 64 MB
 
 
 def _reference(args):
@@ -125,10 +138,14 @@ def build_flagship(n_clients_per_round=10, users=None, norm="gn", comm="auto", o
                      resident=resident, compute_dtype=compute_dtype)
 
 
-def _settle(server, cuda, torch, max_rounds=40, tol=0.05):
+def _settle(server, cuda, torch, max_rounds=40, tol=0.05, fixed=None):
     """Set-up rounds (not warm-up): run until two consecutive rounds agree within ``tol`` — CUDA-graph capture on every
-    rank, symmetric-memory peer mappings and signal pads, NCCL channel set-up and allocator growth happen here."""
+    rank, symmetric-memory peer mappings and signal pads, NCCL channel set-up and allocator growth happen here.
+    ``fixed`` runs exactly that many rounds instead, so the model the later rounds start from does not depend on timing."""
     import time
+    if fixed is not None:
+        server.run_rounds(fixed)
+        return fixed
     prev, n = None, 0
     while n < max_rounds:
         if cuda:
@@ -145,6 +162,30 @@ def _settle(server, cuda, torch, max_rounds=40, tol=0.05):
     return n
 
 
+def _restore_global_model(server, snapshot):
+    """Copies ``snapshot`` back into the global model in place (its tensors are views of the weight arena that the
+    captured CUDA graphs read) and makes the next round resend the weights to the workers."""
+    import torch
+    with torch.no_grad():
+        for k, v in server.worker_trainer.model.state_dict().items():
+            v.copy_(snapshot[k])
+    server._weights_in_sync = False
+
+
+def _dump_outputs(out_dir, server, loss):
+    """``--dump-outputs``: the last round's train loss and the global model it left behind, as ``out_dir/<name>.npy``."""
+    import numpy as np
+    import torch
+    sd = server.worker_trainer.model.state_dict()
+    flat = torch.cat([t.detach().reshape(-1).float() for t in sd.values() if t.is_floating_point()])
+    if flat.numel() > DUMP_MAX_VALUES:
+        idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), DUMP_MAX_VALUES))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "global_model.npy"), flat.cpu().numpy())
+    np.save(os.path.join(out_dir, "train_loss.npy"), np.asarray([float("nan") if loss is None else float(loss)], np.float64))
+
+
 def main():
     args = parse_args()
     if args.impl == "reference":
@@ -154,6 +195,8 @@ def main():
     import statistics
     import time
     import torch
+    if args.dump_outputs:
+        args.dump_outputs = os.path.abspath(args.dump_outputs)
     os.chdir(ROOT)
     logging.getLogger().setLevel(logging.WARNING)
     spec = TASKS[args.task]
@@ -190,7 +233,10 @@ def main():
 
     server = job.server
     server.begin_training()
-    setup_rounds = _settle(server, cuda, torch)
+    initial_model = None
+    if args.dump_outputs:
+        initial_model = {k: v.detach().clone() for k, v in server.worker_trainer.model.state_dict().items()}
+    setup_rounds = _settle(server, cuda, torch, fixed=SETUP_ROUNDS_FIXED if args.dump_outputs else None)
     server.run_rounds(args.warmup)
     Server.sync_nodes({"phases": True})                          # barrier + device synchronize on every rank
     PHASES.enable(True)
@@ -204,7 +250,9 @@ def main():
     t0 = time.perf_counter()
     loss = None
     host_marks = [t0]
-    for _ in range(args.steps):
+    for step in range(args.steps):
+        if initial_model is not None and step == args.steps - 1:
+            _restore_global_model(server, initial_model)
         loss = server.run_rounds(1)
         host_marks.append(time.perf_counter())
         if cuda:
@@ -224,6 +272,8 @@ def main():
     per_round = [marks[i].elapsed_time(marks[i + 1]) for i in range(len(marks) - 1)] if cuda else []
     my_phases = PHASES.totals() if cuda else {}
     PHASES.enable(False)
+    if args.dump_outputs:
+        _dump_outputs(args.dump_outputs, server, loss)
 
     # End-to-end variant: every engine streams its clients' shards host(pinned)->device inside the timed region and the
     # per-round record table is read back (it always is); timed by wall clock around the public run_rounds() call.

@@ -10,16 +10,15 @@ from msrflute_b200.core.schema import SCHEMA
 from msrflute_b200.core.validator import Validator
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# The configs shipped by the original FLUTE (microsoft/msrflute @ 8bfe0854), same layout: they must keep validating.
+REF_CONFIGS = os.path.join(ROOT, "tests", "golden", "reference_configs")
 
 
 def _yamls():
-    pats = [os.path.join(ROOT, "experiments", "*", "config.yaml"), os.path.join(ROOT, "configs", "*.yaml"),
-            os.path.join(ROOT, "testing", "*.yaml")]
-    for ref in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(ref):
-            pats += [os.path.join(ref, "experiments", "*", "config.yaml"), os.path.join(ref, "configs", "*.yaml"),
-                     os.path.join(ref, "testing", "*.yaml")]
-            break
+    pats = []
+    for base in (ROOT, REF_CONFIGS):
+        pats += [os.path.join(base, "experiments", "*", "config.yaml"), os.path.join(base, "configs", "*.yaml"),
+                 os.path.join(base, "testing", "*.yaml")]
     out = []
     for p in pats:
         out += sorted(glob.glob(p))
